@@ -50,6 +50,9 @@ sys.path.insert(0, ROOT)
 import numpy as np  # noqa: E402
 
 METRIC = "LLD frames/sec (16kHz, 25ms/10ms)"
+# the shipped openSMILE configurations the workloads run unchanged, stored with the test fixtures
+CONFIG_DIR = os.path.join(ROOT, "tests", "golden", "config")
+DUMP_BYTES = 8 << 20          # --dump-outputs: at most this many bytes per array (6 arrays stay below 64 MB)
 
 
 class Workload:
@@ -206,6 +209,22 @@ def bind_to_gpu_numa_node(local_rank):
         return {"pci": bus, "numa_node": node, "cpus": cpus, "bound": bool(ids)}
     except Exception as e:      # no sysfs entry (container) -> run unbound, say so
         return {"bound": False, "why": str(e)[:80]}
+
+
+def dump_rows(dump_dir, name, rows):
+    """Writes rows ([n, k] float32, a torch tensor or a numpy array) as dump_dir/<name>.npy and the numbers of the rows written as
+    dump_dir/<name>_row_index.npy (float64).  Above DUMP_BYTES a fixed, seeded sample of rows is written, the same rows in every
+    run with the same arguments, so that the outputs of two builds can be compared."""
+    n, k = rows.shape
+    m = min(n, max(1, DUMP_BYTES // (4 * max(k, 1))))
+    idx = np.sort(np.random.default_rng(0).choice(n, size=m, replace=False)) if m < n else np.arange(n)
+    if isinstance(rows, np.ndarray):
+        sample = rows[idx]
+    else:
+        import torch
+        sample = rows[torch.as_tensor(idx, device=rows.device)].cpu().numpy()
+    np.save(os.path.join(dump_dir, name + ".npy"), np.ascontiguousarray(sample, dtype=np.float32))
+    np.save(os.path.join(dump_dir, name + "_row_index.npy"), idx.astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------
@@ -416,7 +435,7 @@ def make_plan(w, local_rank):
     from opensmile_b200 import Plan, Session, components_mfcc12_0_d_a
     if w.key == "mfcc12":
         return Plan(components_mfcc12_0_d_a(float(w.sr)), "lld", device=local_rank)
-    conf = os.path.join(ROOT, "oracle", "_ref", "config", *w.conf.split("/"))
+    conf = os.path.join(CONFIG_DIR, *w.conf.split("/"))
     opt = {w.out_opt.lstrip("-"): "x.htk"}
     sess = Session(conf, options=opt, device=-1)             # conf front end only; the plan below computes
     comps, level = sess.components(float(w.sr), w.nchan)
@@ -461,6 +480,8 @@ def measure(w, args, rank, world, local_rank, dist, steps, with_cpu, sampler=Non
     ev1.record()
     barrier()
     dt_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        dump_rows(args.dump_outputs, w.key + "_lld", d_out)          # the rows of the last timed step
     # kernel times need a sync per step: taken in a separate pass so the timed loop stays free of host synchronisation
     lld_ms, post_ms = [], []
     for _ in range(min(steps, 10)):
@@ -540,7 +561,7 @@ def measure(w, args, rank, world, local_rank, dist, steps, with_cpu, sampler=Non
     return res
 
 
-def measure_summaries(n_utt=1000):
+def measure_summaries(n_utt=1000, dump_dir=None):
     """SURVEY.md 8(f)-3, reported beside the LLD workloads (not a headline number): the shipped summary configurations end to end
     through the session API from host PCM -- LLD plan, rows resident in HBM, cFunctionals instances + glue, one row per utterance
     copied back.  Wall clock around the blocking call (it synchronises), after one warm-up call on the same batch."""
@@ -552,10 +573,9 @@ def measure_summaries(n_utt=1000):
     base = [mixed_pcm(48000, 16000, seed=s) for s in range(8)]
     pcm = np.concatenate([base[i % 8] for i in range(n_utt)])
     off = np.arange(n_utt + 1, dtype=np.int64) * 48000
-    for rel, tag in (("egemaps/v02/eGeMAPSv02.conf", "eGeMAPSv02.conf -csvoutput"), ("compare16/ComParE_2016.conf", "ComParE_2016.conf -csvoutput")):
-        conf = os.path.join(ROOT, "oracle", "_ref", "config", rel)
-        if not os.path.exists(conf):
-            continue
+    for rel, tag, key in (("egemaps/v02/eGeMAPSv02.conf", "eGeMAPSv02.conf -csvoutput", "egemaps"),
+                          ("compare16/ComParE_2016.conf", "ComParE_2016.conf -csvoutput", "compare16")):
+        conf = os.path.join(CONFIG_DIR, rel)
         try:
             s = Session(conf, options={"csvoutput": "x.csv"}, device=0)
             s.extract_pcm(pcm, off, 16000.0, 1)                  # warm-up with the same batch: buffers sized, modules loaded
@@ -563,6 +583,8 @@ def measure_summaries(n_utt=1000):
             rows, _ = s.extract_pcm(pcm, off, 16000.0, 1)
             dt = time.perf_counter() - t0
             s.close()
+            if dump_dir:
+                dump_rows(dump_dir, "summary_" + key, rows)
             out.append({"config": tag, "utterances": n_utt, "seconds_of_audio": 3.0 * n_utt, "values_per_utterance": int(rows.shape[1]),
                         "wall_s": dt, "utterances_per_s": n_utt / dt, "api": "osm_b200_session_extract_pcm (host PCM in, summary rows out)"})
         except Exception as e:      # a reported extra: never takes the bench line down
@@ -588,7 +610,7 @@ def run_ours(args, rank, world, local_rank):
             if r is not None:
                 others.append({k: r[k] for k in ("value", "unit", "ms_per_step", "steps", "config", "e2e", "gpu_launches", "roofline",
                                                  "parity", "cpu_baseline") if k in r})
-    summaries = measure_summaries() if (world == 1 and not args.no_others and args.workload == "mfcc12") else []
+    summaries = measure_summaries(dump_dir=args.dump_outputs) if (world == 1 and not args.no_others and args.workload == "mfcc12") else []
     if rank == 0:
         line["config"]["numa"] = numa
         if others:
@@ -618,7 +640,15 @@ def main():
                          "plp44k = configs[4] (44.1 kHz stereo)")
     ap.add_argument("--no-others", action="store_true", default=os.environ.get("OSM_BENCH_NO_OTHERS") == "1",
                     help="mfcc12 only: do not append the short measurements of the other three configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the rows the timed path computed in its last step as DIR/<workload>_lld.npy (float32; a fixed, "
+                         "seeded sample of at most 8 MB per array, row numbers in DIR/<name>_row_index.npy) and the summary rows "
+                         "as DIR/summary_<config>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))

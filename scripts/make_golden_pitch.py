@@ -7,7 +7,8 @@ For each case (inputs are regenerated in the tests from opensmile_b200.synth):
                   (level lld ; lld_de, float32 exact)
   <case>_shs/_vit/_sel/_jit/_nz/_nzde/_e60   level taps of tests/configs/compare_pitch_taps.conf (cPitchShs,
                   cPitchSmootherViterbi, cValbasedSelector, cPitchJitter, smoothed level and its delta, rms energy)
-  names_lld       element names of the LLD CSV header; v32k_lld_csv / v32k_lld_arff = the reference's -lldcsvoutput / -lldarffoutput files (-instname utt7) as bytes
+  names_lld       element names of the LLD CSV header; v32k_lld_csv / v32k_lld_arff = the reference's -lldcsvoutput / -lldarffoutput files (-instname utt7) as bytes,
+                  stored in tests/golden/lld_sink_files.npz
 Cases: v32k = voiced_pcm(32000, seed=7); m48k = mixed_pcm(48000, seed=2) (Viterbi lag 1); m30k = mixed_pcm(30000, seed=4);
        m64k = mixed_pcm(64000, seed=3); m60k_44k = mixed_pcm(60000, seed=5) written as a 44.1 kHz file (FFT 4096 / 1024,
        _lld only); m40k_stereo = stereo_mixed_pcm(40000, seed=9), 16 kHz, 2 channels (_lld only); var_m48k / var_m40k = tests/configs/pitch_variants.conf on mixed_pcm(48000, seed=6) / mixed_pcm(40000, seed=8)
@@ -95,7 +96,10 @@ def main():
             out[name + "_lld"] = refrun.read_htk(os.path.join(d, "o.htk"))[0]
             hdr = open(os.path.join(d, "o.csv")).readline().strip().split(";")
             out["names_var"] = np.array([h for h in hdr if h not in ("name", "frameIndex", "frameTime")])
+    # the two sink files go to an archive of their own: each file under tests/golden/ stays below 1 MB
+    sinks = {k: out.pop(k) for k in ("v32k_lld_csv", "v32k_lld_arff")}
     np.savez_compressed(os.path.join(ROOT, "tests", "golden", "pitch_goldens.npz"), **out)
+    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "lld_sink_files.npz"), **sinks)
 
 
 if __name__ == "__main__":

@@ -11,7 +11,7 @@ from oracle import functionals_oracle as fo
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REFCONF = os.path.join(ROOT, "oracle", "_ref", "config")
+REFCONF = os.path.join(HERE, "golden", "config")
 G = np.load(os.path.join(HERE, "golden", "functionals_goldens.npz"))
 G2 = np.load(os.path.join(HERE, "golden", "functionals_goldens2.npz"))
 S, SEC, FR = fo.SEGMENT, fo.SECOND, fo.FRAME
@@ -202,7 +202,6 @@ def _session(conf, opts):
     return Session(conf, options=opts, device=-1)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFCONF, "is09-13")), reason="reference configuration files not built (make -C oracle ref)")
 def test_shipped_is09_configuration_opens_unchanged():
     s = _session(os.path.join(REFCONF, "is09-13", "IS09_emotion.conf"), {"csvoutput": "f.csv"})
     assert s.element_names() == list(G["is09_func_names"])                              # 384 features, the reference's header
@@ -215,7 +214,6 @@ def test_shipped_is09_configuration_opens_unchanged():
     s.close()
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFCONF, "is09-13")), reason="reference configuration files not built (make -C oracle ref)")
 def test_variant_configuration_names(tmp_path):
     conf = tmp_path / "v.conf"
     conf.write_text(open(os.path.join(HERE, "configs", "func_variants.conf")).read().replace("REFCONF", REFCONF))
@@ -225,7 +223,6 @@ def test_variant_configuration_names(tmp_path):
         s.close()
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFCONF, "is09-13")), reason="reference configuration files not built (make -C oracle ref)")
 def test_second_variant_configuration_names(tmp_path):
     conf = tmp_path / "v.conf"
     conf.write_text(open(os.path.join(HERE, "configs", "func_variants2.conf")).read().replace("REFCONF", REFCONF))
@@ -235,7 +232,6 @@ def test_second_variant_configuration_names(tmp_path):
         s.close()
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFCONF, "is09-13")), reason="reference configuration files not built (make -C oracle ref)")
 def test_unimplemented_functionals_are_refused_loudly(tmp_path):
     from opensmile_b200.session import SessionError
     from opensmile_b200 import capi
@@ -264,7 +260,6 @@ def test_unimplemented_functionals_are_refused_loudly(tmp_path):
 GGF = np.load(os.path.join(HERE, "golden", "gemaps_func.npz"))
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFCONF, "egemaps")), reason="reference configuration files not built (make -C oracle ref)")
 @pytest.mark.parametrize("conf,tag", [("egemaps/v02/eGeMAPSv02.conf", "egemaps"), ("gemaps/v01b/GeMAPSv01b.conf", "gemaps")])
 def test_gemaps_summary_names(conf, tag):
     """the shipped GeMAPS / eGeMAPS files open unchanged with -csvoutput: cVectorConcat / cDataSelector (newNames) / cVectorOperation
@@ -337,7 +332,6 @@ def _csv_close(got_text, ref_text, rtol):
         assert np.all(np.abs(va - vb) <= rtol * (np.abs(vb) + 1e-6)), (a[:80], b[:80])
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFCONF, "egemaps")), reason="reference configuration files not built (make -C oracle ref)")
 def test_summary_rows_are_written_like_the_reference_sink(tmp_path):
     """osm_b200_session_write_files on a cFunctionals session: the sink's file has the summary's names, one row per input,
     `'unknown';0.000000;values` -- the reference's file for the same input (the values here are the reference's own, re-printed)"""
@@ -354,17 +348,13 @@ MORE = [("is09-13/IS12_speaker_trait.conf", "IS12_speaker_trait", 5757), ("is09-
         ("gemaps/v01a/GeMAPSv01a.conf", "GeMAPSv01a", 62)]
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFCONF, "is09-13")), reason="reference configuration files not built (make -C oracle ref)")
 @pytest.mark.parametrize("conf,tag,n", MORE)
 def test_more_shipped_summary_configurations_open_with_the_reference_names(conf, tag, n):
-    if not os.path.exists(os.path.join(REFCONF, conf)):
-        pytest.skip("not among the configuration files copied next to the oracle build")
     s = _session(os.path.join(REFCONF, conf), {"csvoutput": "x.csv"})
     assert s.element_names() == [str(x) for x in GMS["names_" + tag]] and len(s.element_names()) == n
     s.close()
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFCONF, "is09-13")), reason="reference configuration files not built (make -C oracle ref)")
 def test_sub_window_functionals_are_refused(tmp_path):
     """the reference's default frameMode is "fixed": a cFunctionals section without frameMode = full summarises sub-windows (the
     MediaEval configurations: frameSize = 2.0) -- refused by name instead of silently summarising the whole input"""

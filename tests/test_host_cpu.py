@@ -89,9 +89,9 @@ def test_no_gpu_means_loud_failure_not_fallback():
         Plan(components_mfcc12_0_d_a(16000.0), "lld", device=0)
 
 
-def test_fft_butterflies_host_build():
+def test_fft_butterflies_host_build(tmp_path):
     """fft_radix.cuh compiled for the host and checked against a naive DFT."""
-    exe = "/tmp/osm_test_fft_radix"
+    exe = str(tmp_path / "test_fft_radix")
     subprocess.check_call(["nvcc", "-std=c++17", "-O2", "-Wno-deprecated-gpu-targets", "-o", exe,
                            os.path.join(ROOT, "tests", "native", "test_fft_radix.cu")])
     subprocess.check_call([exe])
@@ -127,10 +127,10 @@ def test_div32767_trick():
         assert q1 == f32(x / D), k
 
 
-def test_text_sink_number_formatting_equals_printf():
+def test_text_sink_number_formatting_equals_printf(tmp_path):
     """the text sinks format values with std::to_chars into a buffer (opensmile_b200/host/front.cpp TextBuf); for finite
     floats that is byte-identical to the reference's fprintf("%e") / ("%.0f"): 40 M values incl. random bit patterns"""
-    exe = "/tmp/osm_test_fmt_check"
+    exe = str(tmp_path / "fmt_check")
     subprocess.check_call(["g++", "-O2", "-std=c++17", "-o", exe, os.path.join(ROOT, "tests", "native", "fmt_check.cpp")])
     subprocess.check_call([exe], stdout=subprocess.DEVNULL)
 

@@ -1,5 +1,5 @@
 """CPU tests: the oracle (plain-C restatement) against the golden vectors produced by the
-unmodified reference, and -- when oracle/_ref is built -- against the reference itself."""
+unmodified reference."""
 import os
 
 import numpy as np
@@ -7,9 +7,28 @@ import pytest
 
 from conftest import GOLD, rel_to_frame_scale
 from opensmile_b200.synth import voiced_pcm
-from oracle import oracle, refrun
+from oracle import oracle
 
 TOL = 1e-5   # of the per-frame vector scale (north_star: 1e-5 relative, float32)
+# (sample rate, samples, seed, channels) of the inputs whose reference rows tests/golden/reference_rows.npz holds
+# (scripts/make_golden_reference_runs.py)
+MFCC_CASES = [(16000, 40000, 3, 1), (44100, 30000, 4, 1), (16000, 400, 5, 1), (16000, 561, 6, 1), (16000, 20000, 7, 2)]
+PLP_CASES = [(16000, 30000, 11, 1), (44100, 20000, 12, 2), (16000, 560, 13, 1)]
+
+
+def mfcc_key(sr, n, seed, nch):
+    return "mfcc_%d_%d_%d" % (sr, n, seed) + ("_%dch" % nch if nch > 1 else "")
+
+
+def plp_key(sr, n, seed, nch):
+    return "plp_%d_%d_%d_%dch" % (sr, n, seed, nch)
+
+
+def reference_rows(key, pcm):
+    """the unmodified reference's rows for `pcm`, stored under `key`"""
+    g = np.load(os.path.join(GOLD, "reference_rows.npz"))
+    assert int(pcm.astype(np.int64).sum()) == int(g["crc_" + key]), "synthetic generator drifted"
+    return g[key]
 
 
 def test_geometry_known_answers():
@@ -64,20 +83,18 @@ def test_delta_is_bit_exact_on_reference_statics():
         assert np.array_equal(dd[:T], lld[:, 26:39])
 
 
-@pytest.mark.skipif(not refrun.available(), reason="oracle/_ref not built (make -C oracle ref)")
 @pytest.mark.parametrize("sr,n,seed", [(16000, 40000, 3), (44100, 30000, 4), (16000, 400, 5), (16000, 561, 6)])
 def test_oracle_vs_live_reference(sr, n, seed):
     pcm = voiced_pcm(n, sr, seed=seed)
-    ref = refrun.extract("mfcc/MFCC12_0_D_A.conf", pcm, sr)
+    ref = reference_rows(mfcc_key(sr, n, seed, 1), pcm)
     out = oracle.mfcc_d_a(pcm, float(sr))
     assert out.shape == ref.shape
     assert rel_to_frame_scale(out, ref) < TOL
 
 
-@pytest.mark.skipif(not refrun.available(), reason="oracle/_ref not built")
 def test_oracle_vs_live_reference_stereo():
     pcm = voiced_pcm(20000, 16000, seed=7, n_chan=2)
-    ref = refrun.extract("mfcc/MFCC12_0_D_A.conf", pcm, 16000, n_chan=2)
+    ref = reference_rows(mfcc_key(16000, 20000, 7, 2), pcm)
     out = oracle.mfcc_d_a(pcm, 16000.0, n_chan=2)
     assert out.shape == ref.shape
     assert rel_to_frame_scale(out, ref) < TOL
@@ -96,11 +113,10 @@ def test_plp_oracle_vs_golden():
     assert rel_to_frame_scale(out2, g["stereo44k1_lld"]) < TOL
 
 
-@pytest.mark.skipif(not refrun.available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("sr,n,seed,nch", [(16000, 30000, 11, 1), (44100, 20000, 12, 2), (16000, 560, 13, 1)])
+@pytest.mark.parametrize("sr,n,seed,nch", PLP_CASES)
 def test_plp_oracle_vs_live_reference(sr, n, seed, nch):
     pcm = voiced_pcm(n, sr, seed=seed, n_chan=nch)
-    ref = refrun.extract("plp/PLP_0_D_A.conf", pcm, sr, n_chan=nch)
+    ref = reference_rows(plp_key(sr, n, seed, nch), pcm)
     out = oracle.plp_d_a(pcm, float(sr), n_chan=nch)
     assert out.shape == ref.shape
     assert rel_to_frame_scale(out, ref) < TOL

@@ -11,6 +11,7 @@ from oracle import oracle
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 G = np.load(os.path.join(HERE, "golden", "pitch_goldens.npz"))
+SINKS = np.load(os.path.join(HERE, "golden", "lld_sink_files.npz"))
 
 CASES = {
     "v32k": lambda: voiced_pcm(32000, 16000, seed=7),
@@ -96,12 +97,7 @@ def test_compare16_conf_description():
     """The shipped ComParE_2016.conf opens unchanged (sinks without a file name and the functionals they feed
     stay idle); element names and row counts equal the reference's LLD file."""
     from opensmile_b200.session import Session
-    conf = os.path.join(HERE, "configs", "ref", "compare16", "ComParE_2016.conf")
-    if not os.path.exists(conf):
-        from oracle import refrun
-        if not refrun.available():
-            pytest.skip("reference configuration files not available")
-        conf = os.path.join(refrun.CONFIG_DIR, "compare16", "ComParE_2016.conf")
+    conf = _compare16_conf()
     s = Session(conf, options={"lldcsvoutput": "x.csv"}, device=-1)
     assert list(s.element_names(16000.0, 1)) == [str(x) for x in G["names_lld"]]
     off = s.frame_offsets(np.array([0, 32000, 32000 + 48000, 32000 + 48000 + 960]), 16000.0)
@@ -130,13 +126,7 @@ def test_variant_conf_description():
 
 
 def _compare16_conf():
-    conf = os.path.join(HERE, "configs", "ref", "compare16", "ComParE_2016.conf")
-    if os.path.exists(conf):
-        return conf
-    from oracle import refrun
-    if not refrun.available():
-        pytest.skip("reference configuration files not available")
-    return os.path.join(refrun.CONFIG_DIR, "compare16", "ComParE_2016.conf")
+    return os.path.join(HERE, "golden", "config", "compare16", "ComParE_2016.conf")
 
 
 def test_compare16_sink_selection():
@@ -271,7 +261,7 @@ def test_compare16_lld_csv_file_is_byte_identical():
         path = os.path.join(d, "lld.csv")
         write_csv(path, G["v32k_lld"], [str(x) for x in G["names_lld"]], 0.01, instance_name="utt7", frame_index=False,
                   frame_time=True, n_time_frames=p.num_time_frames(32000))
-        assert open(path, "rb").read() == G["v32k_lld_csv"].tobytes()
+        assert open(path, "rb").read() == SINKS["v32k_lld_csv"].tobytes()
     p.close()
     s.close()
 
@@ -285,7 +275,7 @@ def test_compare16_lld_arff_file_is_byte_identical(tmp_path):
     p = tmp_path / "lld.arff"
     write_arff(p, G["v32k_lld"], names, 0.01, relation="openSMILE_features", instance_name="utt7", frame_index=False,
                frame_time=True, classes=(("class", "numeric", "?"),), n_time_frames=195)
-    ref = G["v32k_lld_arff"].tobytes()
+    ref = SINKS["v32k_lld_arff"].tobytes()
     assert p.read_bytes() == ref
     write_arff(p, G["v32k_lld"][:3], names, 0.01, relation="openSMILE_features", instance_name="utt8", frame_index=False,
                frame_time=True, classes=(("class", "numeric", "?"),), append=True)

@@ -12,7 +12,7 @@ from opensmile_b200 import Session, SessionError, capi, write_csv, write_htk
 
 CONF = os.path.join(ROOT, "tests", "configs")
 GOLD = np.load(os.path.join(ROOT, "tests", "golden", "conf_goldens.npz"))
-REF_CONF = os.path.join(ROOT, "oracle", "_ref", "config")
+REF_CONF = os.path.join(ROOT, "tests", "golden", "config")
 
 
 @pytest.mark.parametrize("conf,key", [("lld_mix.conf", "mix"), ("mfcc_e_d_a.conf", "mfcc_e"), ("plp_e_d_a.conf", "plp_e"),
@@ -128,7 +128,6 @@ def test_description_only_session_refuses_to_compute():
     assert e.value.status == capi.ERR_CUDA            # no CPU fallback
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CONF), reason="reference configs not built into oracle/_ref")
 @pytest.mark.parametrize("conf,n", [("mfcc/MFCC12_0_D_A.conf", 39), ("mfcc/MFCC12_E_D_A.conf", 39),
                                     ("plp/PLP_0_D_A.conf", 18), ("plp/PLP_E_D_A.conf", 18),
                                     ("mfcc/MFCC12_0_D_A_Z.conf", 39), ("mfcc/MFCC12_E_D_A_Z.conf", 39),
@@ -256,9 +255,7 @@ def test_parallel_file_sinks_equal_the_single_file_writers(tmp_path):
 def test_inputs_sharing_one_output_file_are_written_in_order(tmp_path):
     """the LLD ARFF sink of the feature-set configurations appends (append = 1): several inputs naming the same file must be
     written one after the other in input order, not by the parallel writers"""
-    ref = os.path.join(ROOT, "oracle", "_ref", "config", "compare16", "ComParE_2016.conf")
-    if not os.path.exists(ref):
-        pytest.skip("reference configuration files not built (make -C oracle ref)")
+    ref = os.path.join(REF_CONF, "compare16", "ComParE_2016.conf")
     s = Session(ref, options={"lldarffoutput": "x.arff", "instname": "u"}, device=-1)
     assert "append=1" in s.sink_options()
     K = len(s.element_names())
@@ -302,8 +299,6 @@ def test_partial_file_options_are_refused_not_ignored():
     """cWaveSource.start / end / endrel select a part of the input file in the reference (iocore/waveSource.cpp:48-58); whole files
     are read here, so any value but the defaults is an error instead of a silently different result"""
     conf = os.path.join(REF_CONF, "mfcc", "MFCC12_0_D_A.conf")
-    if not os.path.exists(conf):
-        pytest.skip("reference configs not built into oracle/_ref")
     Session(conf, options={"O": "x.htk", "start": "0", "end": "-1"}, device=-1).close()
     for opts, needle in (({"start": "1.5"}, "start"), ({"end": "2.0"}, "end")):
         with pytest.raises(SessionError) as e:

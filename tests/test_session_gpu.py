@@ -20,6 +20,7 @@ from opensmile_b200.synth import voiced_pcm
 pytestmark = pytest.mark.gpu
 CONF = os.path.join(ROOT, "tests", "configs")
 GOLD = np.load(os.path.join(ROOT, "tests", "golden", "conf_goldens.npz"))
+REFCONF = os.path.join(ROOT, "tests", "golden", "config")
 
 
 def col_err(got, ref):
@@ -215,22 +216,16 @@ def test_cepstral_mean_subtraction_confs():
         assert got.shape == ref.shape
         assert (np.abs(got - ref) / np.abs(GOLD["mfcc_z_plain"]).max(axis=1, keepdims=True)).max() < 1e-5
     assert np.array_equal(rows[fo[0]:fo[1]], rows[fo[2]:fo[3]])
-    refdir = os.path.join(ROOT, "oracle", "_ref", "config")
-    if os.path.isdir(refdir):
-        for key, rel in (("ref_mfcc_0_z", "mfcc/MFCC12_0_D_A_Z.conf"), ("ref_mfcc_e_z", "mfcc/MFCC12_E_D_A_Z.conf"),
-                         ("ref_plp_0_z", "plp/PLP_0_D_A_Z.conf"), ("ref_plp_e_z", "plp/PLP_E_D_A_Z.conf")):
-            s = Session(os.path.join(refdir, rel))
-            got, _ = s.extract_pcm(pcm, [0, 12000], 16000, 1)
-            ref = GOLD[key]
-            assert got.shape == ref.shape, key
-            # scale: the un-normalised statics are ~1e1, mean-subtracted columns can be ~0 in a whole row
-            assert np.abs(got - ref).max() < 1e-5 * np.abs(ref).max(), key
+    for key, rel in (("ref_mfcc_0_z", "mfcc/MFCC12_0_D_A_Z.conf"), ("ref_mfcc_e_z", "mfcc/MFCC12_E_D_A_Z.conf"),
+                     ("ref_plp_0_z", "plp/PLP_0_D_A_Z.conf"), ("ref_plp_e_z", "plp/PLP_E_D_A_Z.conf")):
+        s = Session(os.path.join(REFCONF, rel))
+        got, _ = s.extract_pcm(pcm, [0, 12000], 16000, 1)
+        ref = GOLD[key]
+        assert got.shape == ref.shape, key
+        # scale: the un-normalised statics are ~1e1, mean-subtracted columns can be ~0 in a whole row
+        assert np.abs(got - ref).max() < 1e-5 * np.abs(ref).max(), key
 
 
-REFCONF = os.path.join(ROOT, "oracle", "_ref", "config")
-
-
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFCONF, "audspec")), reason="reference configs not built into oracle/_ref")
 def test_more_shipped_configs_audspec_spectrogram_demo1(tmp_path):
     """config/audspec/*.conf (auditory spectrum + deltas), config/spectrum/spectrogram.conf (the magnitude
     level itself as output) and config/demo/demo1_energy.conf (CSV sink with a frame index column), unchanged."""

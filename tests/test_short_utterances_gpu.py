@@ -14,13 +14,12 @@ from opensmile_b200.synth import voiced_pcm
 
 pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
-REFCONF = os.path.join(HERE, "..", "oracle", "_ref", "config")
+REFCONF = os.path.join(HERE, "golden", "config")
 G = np.load(os.path.join(HERE, "golden", "short_utterances.npz"))
 LENS = (900, 1000, 1130, 1290, 1450, 1610, 2000, 3000, 4800)
 SEG_DE = ["F0final_sma_de", "voicingFinalUnclipped_sma_de", "jitterLocal_sma_de", "jitterDDP_sma_de", "shimmerLocal_sma_de", "logHNR_sma_de"]
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFCONF, "compare16")), reason="reference configuration files not built (make -C oracle ref)")
 @pytest.mark.parametrize("conf,tag", [("compare16/ComParE_2016.conf", "c16"), ("egemaps/v02/eGeMAPSv02.conf", "ege")])
 def test_short_utterances(conf, tag):
     from opensmile_b200.session import Session

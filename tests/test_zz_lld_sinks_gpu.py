@@ -13,7 +13,8 @@ from opensmile_b200.synth import voiced_pcm
 pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
 G = np.load(os.path.join(HERE, "golden", "pitch_goldens.npz"))
-CONF = os.path.join(os.path.dirname(HERE), "oracle", "_ref", "config", "compare16", "ComParE_2016.conf")
+SINKS = np.load(os.path.join(HERE, "golden", "lld_sink_files.npz"))
+CONF = os.path.join(HERE, "golden", "config", "compare16", "ComParE_2016.conf")
 
 
 def _write_wav(path, pcm, sr):
@@ -27,8 +28,6 @@ def _write_wav(path, pcm, sr):
 
 def test_compare16_three_lld_sinks(tmp_path):
     from opensmile_b200.session import Session
-    if not os.path.exists(CONF):
-        pytest.skip("reference configuration files not built (make -C oracle ref)")
     wav = tmp_path / "in.wav"
     _write_wav(wav, voiced_pcm(32000, 16000, seed=7), 16000)
     s = Session(CONF, options={"lldcsvoutput": "x.csv", "lldarffoutput": "x.arff", "lldhtkoutput": "x.htk", "instname": "utt7"}, device=0)
@@ -40,7 +39,7 @@ def test_compare16_three_lld_sinks(tmp_path):
 
     # CSV: same header, same name / time columns, values within tolerance (printed with 7 significant digits)
     got = (tmp_path / "o.csv").read_text().splitlines()
-    exp = G["v32k_lld_csv"].tobytes().decode().splitlines()
+    exp = SINKS["v32k_lld_csv"].tobytes().decode().splitlines()
     assert got[0] == exp[0] and len(got) == len(exp)
     for a, b in zip(got[1:], exp[1:]):
         fa, fb = a.split(";"), b.split(";")
@@ -49,7 +48,7 @@ def test_compare16_three_lld_sinks(tmp_path):
 
     # ARFF: identical header block, identical name / time / target fields
     got = (tmp_path / "o.arff").read_text().split("\n")
-    exp = G["v32k_lld_arff"].tobytes().decode().split("\n")
+    exp = SINKS["v32k_lld_arff"].tobytes().decode().split("\n")
     n_hdr = exp.index("@data") + 2
     assert got[:n_hdr] == exp[:n_hdr] and len(got) == len(exp)
     for a, b in zip(got[n_hdr:-1], exp[n_hdr:-1]):

@@ -12,7 +12,7 @@ from opensmile_b200.synth import mixed_pcm
 
 pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.path.join(os.path.dirname(HERE), "oracle", "_ref", "config")
+REF = os.path.join(HERE, "golden", "config")
 TOL = 1e-5
 
 
@@ -24,8 +24,6 @@ def _percol(got, ref):
                                            ("egemaps/v02/eGeMAPSv02.conf", {"lldcsvoutput": "x.csv"}, "egemaps_lld")])
 def test_shipped_configuration_rows(conf, opts, key):
     from opensmile_b200.session import Session
-    if not os.path.isdir(REF):
-        pytest.skip("reference configuration files not built (make -C oracle ref)")
     G = np.load(os.path.join(HERE, "golden", "formant_goldens.npz"))
     pcms = [mixed_pcm(24000, 16000, seed=3), mixed_pcm(40000, 16000, seed=5)]
     off = np.concatenate([[0], np.cumsum([len(x) for x in pcms])]).astype(np.int64)
@@ -44,8 +42,6 @@ def test_shipped_configuration_rows(conf, opts, key):
 def test_all_shipped_gemaps_family_rows():
     """the five shipped feature-set files (v01a / v01b / v02) against the reference's LLD rows (tests/golden/gemaps_family.npz)"""
     from opensmile_b200.session import Session
-    if not os.path.isdir(REF):
-        pytest.skip("reference configuration files not built (make -C oracle ref)")
     gold = json.load(open(os.path.join(HERE, "golden", "gemaps_headers.json")))
     R = np.load(os.path.join(HERE, "golden", "gemaps_family.npz"))
     pcm = mixed_pcm(24000, 16000, seed=3)
